@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """Benchmark of the fused D3PM reverse-diffusion token update (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+
+`--steps` sets the timed steps of the headline metric.  `--dump-outputs DIR` (`--impl ours` only) writes the tokens of
+the last timed step to DIR/x_prev.npy.
 
 A "step" is ONE fused reverse step (classifier-free guidance + posterior + Gumbel-max sample, production
 in-kernel Philox mode) over one batch of synthetic logits.  Workload at N GPUs: BASELINE config 2 per GPU
@@ -322,6 +325,8 @@ def run_ours(args):
     elapsed_ms = ev0.elapsed_time(ev1)
     assert int(status.item()) & (_lib.STATUS_BAD_T | _lib.STATUS_BAD_TOKEN) == 0
     assert int(x_prev.min()) >= 0 and int(x_prev.max()) <= K
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x_prev, B_global, rank)
 
     # ---- config 4's claim on hardware: the gathered tokens of the sharded job equal what ONE GPU computes for the same
     # global videos.  One step at a fixed offset on every rank, the (timed) token all-gather, then rank 0 regenerates
@@ -484,6 +489,25 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, x_prev, B_global, rank):
+    """Write what the last timed step returned to its caller, the sampled tokens x_{t-1} of the whole job, as
+    `out_dir/x_prev.npy` (float64 [videos, tokens], token ids are exact).  The inputs, the Philox seed and the offset of the
+    last step depend only on the arguments, so two builds run with the same arguments can be compared token for token.
+    A job larger than 64 MB of such tokens is written as a fixed, seeded sample of whole videos, in video order."""
+    import numpy as np
+    import torch
+
+    import d3pm_b200
+    tokens = d3pm_b200.gather_tokens(x_prev, B_global)  # every rank takes part in the all-gather
+    max_videos = (64 << 20) // (8 * tokens.shape[1])
+    if tokens.shape[0] > max_videos:
+        keep = torch.randperm(tokens.shape[0], generator=torch.Generator().manual_seed(0))[:max_videos].sort().values
+        tokens = tokens[keep.to(tokens.device)]
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "x_prev.npy"), tokens.cpu().numpy().astype(np.float64))
 
 
 def _timed_steps(fn, n, dev, warm=3):
@@ -774,14 +798,21 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=300,
-                    help="timed steps; the default (0.1 s) is a burst measurement like MEASURED_PEAKS.json's copy "
-                         "bandwidth, the `sustained` block of the line reports a 1500-step run (power-capped on B200)")
+                    help="timed steps of the headline metric (`value`, `ms_per_step`); the default (0.1 s) is a burst "
+                         "measurement.  The other blocks keep their own counts, reported beside them: `e2e` times "
+                         "min(steps, 10) steps (at least 3), `sustained` a fixed 1500 (power-capped on B200)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--global-videos", type=int, default=0,
                     help="strong scaling: this many videos in total, split over the ranks (config 4: 128); "
                          "default 0 = weak scaling, 16 videos per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the tokens the last timed step sampled to DIR/x_prev.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the tokens of --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

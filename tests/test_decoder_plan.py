@@ -9,9 +9,9 @@ import numpy as np
 import pytest
 import torch
 
-from baseline import reference_loader as RL
 from d3pm_b200 import decode
 from oracle import decoder_oracle as DO
+from tests.helpers import vqvae_from_fixture
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -100,15 +100,11 @@ def run_plan(plan, h):
             return emulate_col2im(emulate_conv(item[1], x, B, grid), item[3], B, grid, item[4], item[2])
 
 
-@pytest.mark.skipif(not RL.reference_available(), reason="the plan is read off the reference's Decoder module")
 @pytest.mark.parametrize("name", ["decode_h64", "decode_h128", "decode_small", "decode_k512"])   # the last two: n_hiddens 24, padded to 64
 def test_plan_through_the_kernel_contracts_reproduces_the_reference_video(name):
     fx = np.load(os.path.join(GOLD, name + ".npz"))
-    E, K, Hd, R, d0, d1, d2, L, res, B = (int(v) for v in fx["hparams"])
-    vq = RL.load_vqvae_module().VQVAE(checkpoint_path=None, embedding_dim=E, n_codes=K, n_hiddens=Hd, n_res_layers=R,
-                                      downsample=[d0, d1, d2], sequence_length=L, resolution=res)
-    vq.load_state_dict({k[3:]: torch.from_numpy(fx[k]) for k in fx.files if k.startswith("sd/")}, strict=False)
-    plan = decode.decoder_plan(vq.eval().decoder)
+    vq = vqvae_from_fixture(fx)
+    plan = decode.decoder_plan(vq.decoder)
     got = run_plan(plan, torch.from_numpy(fx["h"]))
     want = torch.from_numpy(fx["video"])
     assert got.shape == want.shape

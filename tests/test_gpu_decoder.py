@@ -11,6 +11,7 @@ from baseline import reference_loader as RL
 from d3pm_b200 import _lib, decode, ops
 from d3pm_b200._lib import D3PMError
 from oracle import decoder_oracle as DO
+from tests.helpers import reference_vqvae_like, vqvae_from_fixture, vqvae_layout
 from tests.test_decoder_plan import emulate_attention, emulate_col2im, emulate_conv
 
 pytestmark = pytest.mark.gpu
@@ -117,21 +118,11 @@ def test_col2im(stride):
     assert (out.cpu() - want).abs().max().item() <= 1e-5 * float(want.abs().max())
 
 
-def _vqvae_from_fixture(fx):
-    E, K, Hd, R, d0, d1, d2, L, res, B = (int(v) for v in fx["hparams"])
-    vq = RL.load_vqvae_module().VQVAE(checkpoint_path=None, embedding_dim=E, n_codes=K, n_hiddens=Hd, n_res_layers=R,
-                                      downsample=[d0, d1, d2], sequence_length=L, resolution=res)
-    vq.load_state_dict({k[3:]: torch.from_numpy(fx[k]) for k in fx.files if k.startswith("sd/")}, strict=False)
-    return vq.to(DEV).eval()
-
-
 @pytest.mark.parametrize("name", ["decode_h64", "decode_h128", "decode_small", "decode_k512"])   # the last two: n_hiddens 24, padded to 64
 def test_native_decoder_against_reference_fixture(name):
     """tokens -> video entirely on the library's kernels, against the video the imported reference's `VQVAE.decode` returned."""
-    if not RL.reference_available():
-        pytest.skip("reference not staged (baseline/_ref absent): the decoder plan is read off the reference's module")
     fx = np.load(os.path.join(GOLD, name + ".npz"))
-    vq = _vqvae_from_fixture(fx)
+    vq = vqvae_from_fixture(fx).to(DEV)
     tokens = torch.from_numpy(fx["tokens"]).to(DEV)
     want = torch.from_numpy(fx["video"])
     scale = float(want.abs().max())
@@ -158,43 +149,42 @@ def test_native_decoder_against_reference_fixture(name):
 
 @pytest.mark.parametrize("B", [1, 3])
 def test_native_decoder_at_the_shipped_shape_against_the_live_reference(B):
-    """n_hiddens 256, 3 residual blocks, downsample [1, 8, 8], 4 x 128 x 128 video (ucf-ddiff-train.job:15): the reference's
-    own `VQVAE.decode` on this GPU in fp32 (TF32 off) vs the native chain with the same weights."""
-    if not RL.reference_available():
-        pytest.skip("reference not staged (baseline/_ref absent)")
+    """n_hiddens 256, 3 residual blocks, downsample [1, 8, 8], 4 x 128 x 128 video (ucf-ddiff-train.job:15): the native chain
+    against the oracle (CPU, fp32; pinned to the reference's videos by tests/golden/decode_*.npz), and -
+    where the reference is present - against the reference's own `VQVAE.decode` on this GPU in fp32 (TF32 off), same weights."""
     torch.manual_seed(21)
-    vq = RL.load_vqvae_module().VQVAE(checkpoint_path=None, embedding_dim=128, n_codes=4096, n_hiddens=256, n_res_layers=3,
-                                      downsample=[1, 8, 8], sequence_length=4, resolution=128)
+    vq = vqvae_layout(128, 4096, 256, 3, (1, 8, 8))
     with torch.no_grad():
         for m in vq.modules():
             if isinstance(m, torch.nn.BatchNorm3d):
                 m.running_mean.normal_(0, 0.2)
                 m.running_var.uniform_(0.5, 1.5)
-    vq = vq.to(DEV).eval()
+    vq = vq.to(DEV)
     tokens = torch.randint(0, 4096, (B, 4, 16, 16), device=DEV)
-    tf32_conv, tf32_mm = torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        with torch.no_grad():
-            want = vq.decode(tokens).cpu()
-    finally:
-        torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = tf32_conv, tf32_mm
     table = decode.DecodeTable.from_autoencoder(vq)
     got = decode.decode(vq, tokens, table, decode.NativeDecoder(vq.decoder)).cpu()
-    scale = float(want.abs().max())
-    assert got.shape == want.shape == (B, 3, 4, 128, 128)
-    assert (got - want).abs().max().item() <= 1e-4 * scale
-    # and the oracle (CPU, fp32) on the same weights for one video
+    assert got.shape == (B, 3, 4, 128, 128)
     sd = {k: v.detach().cpu() for k, v in vq.state_dict().items()}
-    orc = DO.vqvae_decode(sd, tokens[:1].cpu(), 3, (1, 8, 8))
-    assert (got[:1] - orc).abs().max().item() <= 1e-4 * scale
+    orc = DO.vqvae_decode(sd, tokens.cpu(), 3, (1, 8, 8))
+    assert (got - orc).abs().max().item() <= 1e-4 * float(orc.abs().max())
+    if RL.reference_available():
+        ref = reference_vqvae_like(vq, embedding_dim=128, n_codes=4096, n_hiddens=256, n_res_layers=3, downsample=[1, 8, 8],
+                                   sequence_length=4, resolution=128)
+        tf32_conv, tf32_mm = torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
+        torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
+        try:
+            with torch.no_grad():
+                want = ref.decode(tokens).cpu()
+        finally:
+            torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = tf32_conv, tf32_mm
+        assert want.shape == got.shape
+        assert (got - want).abs().max().item() <= 1e-4 * float(want.abs().max())
 
 
 def test_sample_then_decode_like_the_reference_caller():
     """`DiscreteDiffusion.forward`'s inference branch (networks/discrete_diffusion.py:53-62): sample the tokens with the drop-in
-    diffusion class, view them on the latent grid, decode - natively and through the reference's own `VQVAE.decode`."""
-    if not RL.reference_available():
-        pytest.skip("reference not staged (baseline/_ref absent)")
+    diffusion class, view them on the latent grid, decode natively - against the oracle's `VQVAE.decode` (CPU, fp32) and,
+    where the reference is present, the reference's own `VQVAE.decode`."""
     import types
     import d3pm_b200
     K, B, grid = 256, 2, (2, 4, 4)
@@ -213,16 +203,21 @@ def test_sample_then_decode_like_the_reference_caller():
     model = d3pm_b200.FusedDiffusionTransformer(transformer=Denoiser(), diffusion_step=20, alpha_init_type="alpha1", guidance_scale=2.0,
                                                 content_seq_len=N).to(DEV)
     torch.manual_seed(5)
-    vq = RL.load_vqvae_module().VQVAE(checkpoint_path=None, embedding_dim=32, n_codes=K, n_hiddens=64, n_res_layers=1,
-                                      downsample=[1, 4, 4], sequence_length=grid[0], resolution=4 * grid[1]).to(DEV).eval()
+    vq = vqvae_layout(32, K, 64, 1, (1, 4, 4)).to(DEV)
     cond = torch.zeros(B, 1, 512, device=DEV)
     video = decode.sample_and_decode(model.manual_seed(3), vq, ["a"] * B, cond, cond, grid, decoder=decode.NativeDecoder(vq.decoder))
     tokens = model.manual_seed(3).sample(["a"] * B, None, cond, cond, content_token=None, filter_ratio=0)["content_token"]
     assert not (tokens == K).any()
-    with torch.no_grad():
-        want = vq.decode(tokens.view(B, *grid))
-    assert video.shape == want.shape == (B, 3, grid[0], 4 * grid[1], 4 * grid[2])
-    assert (video - want).abs().max().item() <= 2e-3 * float(want.abs().max())   # the reference arm runs cuDNN's default TF32 here
+    sd = {k: v.detach().cpu() for k, v in vq.state_dict().items()}
+    orc = DO.vqvae_decode(sd, tokens.view(B, *grid).cpu(), 1, (1, 4, 4))
+    assert video.shape == orc.shape == (B, 3, grid[0], 4 * grid[1], 4 * grid[2])
+    assert (video.cpu() - orc).abs().max().item() <= 1e-4 * float(orc.abs().max())
+    if RL.reference_available():
+        ref = reference_vqvae_like(vq, embedding_dim=32, n_codes=K, n_hiddens=64, n_res_layers=1, downsample=[1, 4, 4],
+                                   sequence_length=grid[0], resolution=4 * grid[1])
+        with torch.no_grad():
+            want = ref.decode(tokens.view(B, *grid))
+        assert (video - want).abs().max().item() <= 2e-3 * float(want.abs().max())   # the reference arm runs cuDNN's default TF32 here
 
 
 @pytest.mark.parametrize("pair", [False, True])
@@ -298,10 +293,8 @@ def test_decoder_kernels_on_a_non_current_device():
 def test_native_decode_can_be_captured_in_a_cuda_graph():
     """Serving loops replay a captured graph: the whole native decode (gather, 3xTF32 GEMMs with cluster launches off and on,
     attention, col2im) records into a CUDA graph and replays to the eager result on new tokens."""
-    if not RL.reference_available():
-        pytest.skip("reference not staged (baseline/_ref absent)")
     fx = np.load(os.path.join(GOLD, "decode_h64.npz"))
-    vq = _vqvae_from_fixture(fx)
+    vq = vqvae_from_fixture(fx).to(DEV)
     table = decode.DecodeTable.from_autoencoder(vq)
     K = int(fx["hparams"][1])
     for pair in (False, True):
