@@ -403,9 +403,8 @@ int d3pm_head_step(const d3pm_head_desc* d) {
   p.seed = d->seed, p.offset = d->offset, p.row_offset = d->row_offset;
   const cudaStream_t s = static_cast<cudaStream_t>(d->stream);
   const bool has_u = d->hidden_u != nullptr;
-  int dev = 0, sms = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-    return fail(D3PM_ERR_CUDA, "head_step: cannot query the device");
+  const int sms = d3pm::host::sm_count();
+  if (sms == 0) return fail(D3PM_ERR_CUDA, "head_step: cannot query the device");
   if (d->mode == D3PM_HEAD_REFERENCE) {
     const unsigned grid = static_cast<unsigned>(rows < 8LL * sms ? rows : 8LL * sms);
     if (has_u) H::head_redo_kernel<64, true><<<grid, H::kRedoThreads, 0, s>>>(p, 1);
@@ -488,18 +487,6 @@ struct d3pm_host_step {
 };
 
 namespace {
-class SetDevice {  // make `dev` current for the scope
- public:
-  explicit SetDevice(int dev) {
-    if (cudaGetDevice(&prev_) == cudaSuccess && prev_ != dev) switched_ = cudaSetDevice(dev) == cudaSuccess;
-  }
-  ~SetDevice() {
-    if (switched_) cudaSetDevice(prev_);
-  }
- private:
-  int prev_ = 0;
-  bool switched_ = false;
-};
 #define D3PM_CUDA_OK(call, what)                                                                   \
   do {                                                                                             \
     const cudaError_t e_ = (call);                                                                 \
@@ -509,7 +496,7 @@ class SetDevice {  // make `dev` current for the scope
 
 extern "C" int d3pm_host_step_destroy(d3pm_host_step* h) {
   if (h == nullptr) return D3PM_OK;
-  const SetDevice on(h->device);
+  const DeviceGuard on_device(h->device);
   if (h->compute != nullptr) cudaStreamSynchronize(h->compute);
   if (h->copy != nullptr) cudaStreamSynchronize(h->copy);
   for (void* ptr : {static_cast<void*>(h->logits_c), static_cast<void*>(h->logits_u), static_cast<void*>(h->hidden_c),
@@ -534,7 +521,7 @@ extern "C" int d3pm_host_step_create(d3pm_host_step** out, int device, int B, in
     return fail(D3PM_ERR_UNSUPPORTED, "host_step_create: B=%d N=%d T=%d must be positive, K=%d in {1024,2048,4096}, D=%d in {0,64}", B, N, T, K, D);
   if (chunks <= 0) chunks = (B % 4 == 0 && static_cast<int64_t>(B) * N / 4 >= 1024) ? 4 : 1;
   if (chunks > 16 || B % chunks != 0) return fail(D3PM_ERR_INVALID, "host_step_create: chunks=%d must divide B=%d and be <= 16", chunks, B);
-  const SetDevice on(device);
+  const DeviceGuard on_device(device);
   d3pm_host_step* h = new d3pm_host_step;
   h->device = device, h->B = B, h->N = N, h->K = K, h->T = T, h->D = D, h->chunks = chunks, h->guidance = guidance != 0;
   const size_t rows = static_cast<size_t>(B) * N;
@@ -585,7 +572,7 @@ extern "C" int64_t d3pm_host_step_d2h_bytes(const d3pm_host_step* h) { return h 
 template <typename Launch>
 static int host_step_run(d3pm_host_step* h, const float* in_c, const float* in_u, float* dev_c, float* dev_u, int64_t width,
                          const int64_t* x_t, const int64_t* t, int64_t* x_prev, uint32_t* status_out, Launch launch, size_t elem = 4) {
-  const SetDevice on(h->device);
+  const DeviceGuard on_device(h->device);
   const size_t rows = static_cast<size_t>(h->B) * h->N;
   D3PM_CUDA_OK(cudaMemcpyAsync(h->x_t, x_t, rows * 8, cudaMemcpyHostToDevice, h->compute), "host_step: x_t copy");
   D3PM_CUDA_OK(cudaMemcpyAsync(h->t, t, static_cast<size_t>(h->B) * 8, cudaMemcpyHostToDevice, h->compute), "host_step: t copy");

@@ -79,9 +79,8 @@ int d3pm_dec_conv(const d3pm_dec_conv_desc* d) {
   const int ctas = d->cta_pair ? 2 : 1;
   const long long mtiles = ((M + D::kTileM - 1) / D::kTileM + ctas - 1) / ctas;
   const long long tiles = mtiles * (p.Npad / d->n_tile) * d->nclass;
-  int dev = 0, sms = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-    return fail(D3PM_ERR_CUDA, "dec_conv: cannot query the device");
+  const int sms = d3pm::host::sm_count();
+  if (sms == 0) return fail(D3PM_ERR_CUDA, "dec_conv: cannot query the device");
   const long long units = tiles < sms / ctas ? tiles : sms / ctas;  // persistent: one CTA (or pair) per SM (TPC) walks the tiles
   const cudaStream_t s = static_cast<cudaStream_t>(d->stream);
   auto launch = [&](auto kern, size_t smem) -> int {

@@ -25,6 +25,7 @@
 #include <stdint.h>
 
 #include "d3pm_b200.h"
+#include "d3pm_ptx.cuh"
 
 namespace d3pm {
 namespace dec {
@@ -56,116 +57,6 @@ struct GemmParams {
   signed char tap[kMaxClasses][kMaxTaps][4];  // (dt, dh, dw) of every tap of every class
   signed char cls[kMaxClasses][4];            // (pt, ph, pw): output position = input position * stride + this
 };
-
-// ---- PTX wrappers ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}"
-      ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(unsigned long long* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tc_mma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// ---- pairs of CTAs (cta_group::2): the leader CTA issues M = 256 MMAs over both CTAs' shared memory and tensor memory
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire;" ::: "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(unsigned long long* bar, uint32_t cta) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(bar)), "r"(cta));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(r) : "memory");
-}
-__device__ __forceinline__ bool mbar_test(unsigned long long* bar, uint32_t parity) {  // non-blocking
-  uint32_t done;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(done)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return done != 0;
-}
-__device__ __forceinline__ void mbar_wait_cluster(unsigned long long* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1, %2;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}"
-      ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680)
-      : "memory");
-}
-__device__ __forceinline__ void tc_commit_pair(unsigned long long* bar) {  // arrives on `bar` in both CTAs of the pair
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(static_cast<unsigned short>(3))
-               : "memory");
-}
-__device__ __forceinline__ void tc_mma_tf32_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// K-major operand, 128-byte swizzle: rows at 128 B, 8-row groups at SBO = 1024 B, descriptor version 1 (sm_100)
-__device__ __forceinline__ uint64_t smem_desc(uint32_t addr) {
-  return static_cast<uint64_t>((addr >> 4) & 0x3fffu) | (static_cast<uint64_t>(1024 >> 4) << 32) | (1ull << 46) | (2ull << 61);
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-        "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-        "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // nearest tf32 number (10 mantissa bits, ties away from zero): the tensor core ignores the 13 low bits, so rounding here makes
 // the single-product mode unbiased; in the 3xTF32 mode lo = x - hi stays exact either way
@@ -217,8 +108,7 @@ struct GemmGeo {
   static constexpr int kABytes = kHalves * kBlockBytes;           // A part of a stage
   static constexpr int kStageBytes = kABytes + kHalves * kBBytes;
   static constexpr int kStages = 196608 / kStageBytes < 6 ? 196608 / kStageBytes : 6;
-  // instruction descriptor: D = f32, A = B = tf32, both K-major, N = NT, M = 128 per CTA
-  static constexpr uint32_t kIdesc = (1u << 4) | (2u << 7) | (2u << 10) | ((NT >> 3) << 17) | (((kTileM * CTAS) >> 4) << 24);
+  static constexpr uint32_t kIdesc = idesc_tf32(kTileM * CTAS, NT);  // M = 128 per CTA
 };
 
 struct GemmCtl {
@@ -269,7 +159,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) conv_gemm_kernel(const __grid
     for (int i = 0; i < G::kStages; ++i)
       mbar_init(&C.full_a[i], kProdThreads), mbar_init(&C.full_b[i], 1), mbar_init(&C.empty[i], 1), mbar_init(&C.peer_full[i], 1);
     for (int i = 0; i < 2; ++i) mbar_init(&C.acc_full[i], 1), mbar_init(&C.acc_empty[i], kEpiWarps * CTAS);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (p.in_scale != nullptr)
     for (int i = tid; i < p.Cin; i += kGemmThreads) C.scale[i] = p.in_scale[i], C.shift[i] = p.in_shift[i];
@@ -279,13 +169,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1) conv_gemm_kernel(const __grid
     C.tap_shift[c][t] = ((p.tap[c][t][0] * p.H + p.tap[c][t][1]) * p.W + p.tap[c][t][2]) * p.Cin;
   }
   if (warp == 0) {  // two accumulators of NT columns (in both CTAs of a pair: the same warp of each allocates)
-    if constexpr (CTAS == 2) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&C.tmem_base)), "n"(2 * NT) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&C.tmem_base)), "n"(2 * NT) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    tmem_alloc<CTAS, 2 * NT>(&C.tmem_base);
+    tmem_relinquish<CTAS>();
   }
   tc_fence_before();
   __syncthreads();
@@ -475,7 +360,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) conv_gemm_kernel(const __grid
           asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a_hi + kBlockBytes + soff[i]), "f"(lo[0]), "f"(lo[1]), "f"(lo[2]), "f"(lo[3])
                        : "memory");
       }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async();
       mbar_arrive(&C.full_a[e_st]);
       if (++e_st == G::kStages) e_st = 0, e_par ^= 1u;
       if (++e_cb == CB) e_cb = 0;
@@ -633,8 +518,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) conv_gemm_kernel(const __grid
   if constexpr (CTAS == 2) cluster_sync();  // both CTAs are done with the pair's tensor memory and barriers
   if (warp == 0) {
     tc_fence_after();
-    if constexpr (CTAS == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(2 * NT) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(2 * NT) : "memory");
+    tmem_dealloc<CTAS, 2 * NT>(tmem);
   }
 }
 

@@ -32,6 +32,8 @@
 
 #include <type_traits>
 
+#include "d3pm_host.h"
+#include "d3pm_ptx.cuh"
 #include "d3pm_step_rows.cuh"
 
 namespace d3pm {
@@ -85,37 +87,6 @@ struct __align__(128) GroupSmem {
   int32_t redo[Sh::RC];
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-// bulk TMA (1-D): global -> shared, completion bytes counted on the mbarrier.  (An L2 evict-first hint was
-// measured ~4 % slower on B200 for this read-once stream, so the copies carry no cache hint.)
-__device__ __forceinline__ void tma_load_row(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
 __device__ __forceinline__ void group_bar(int id) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(kGroupThreads) : "memory");
 }
@@ -372,12 +343,13 @@ __global__ void __launch_bounds__(kStreamThreads, 1) step_stream_kernel(const __
   // issues the copies, and the set-up below (coefficient table into shared memory, list counters) runs under that latency.
   if (tg == 0) {
     mbar_init(&S.full, 1);
+    fence_mbarrier_init();
     S.redo_cnt = 0;
     if (!exact_mode && first_row < rows) {
       const unsigned long long at = static_cast<unsigned long long>(static_cast<uint32_t>(first_row)) * pitch;
       mbar_expect_tx(&S.full, HAS_U ? 2 * kRowBytes : kRowBytes);
-      tma_load_row(S.c, LT::row(p.logits_c, at), kRowBytes, &S.full);
-      if (HAS_U) tma_load_row(S.u, LT::row(p.logits_u, at), kRowBytes, &S.full);
+      tma_load(S.c, LT::row(p.logits_c, at), kRowBytes, &S.full);
+      if (HAS_U) tma_load(S.u, LT::row(p.logits_u, at), kRowBytes, &S.full);
     }
   }
   // CTA-wide copy of the coefficient table (16 floats per timestep) when it fits: per-row lookups become LDS
@@ -394,10 +366,10 @@ __global__ void __launch_bounds__(kStreamThreads, 1) step_stream_kernel(const __
 
   auto issue_row = [&](int row) {  // elected thread: arm the barrier and launch both row copies
     const unsigned long long at = static_cast<unsigned long long>(static_cast<uint32_t>(row)) * pitch;
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    fence_proxy_async();
     mbar_expect_tx(&S.full, HAS_U ? 2 * kRowBytes : kRowBytes);
-    tma_load_row(S.c, LT::row(p.logits_c, at), kRowBytes, &S.full);
-    if (HAS_U) tma_load_row(S.u, LT::row(p.logits_u, at), kRowBytes, &S.full);
+    tma_load(S.c, LT::row(p.logits_c, at), kRowBytes, &S.full);
+    if (HAS_U) tma_load(S.u, LT::row(p.logits_u, at), kRowBytes, &S.full);
   };
   // slot (register chunk index) of the low chunk of coarse call c: chunks q and q + 128 share a call, i.e. slots
   // i and i + PS of the same thread
@@ -419,7 +391,7 @@ __global__ void __launch_bounds__(kStreamThreads, 1) step_stream_kernel(const __
   auto process_row = [&](auto exact_c, int row, int next_row, uint32_t j, int tt, int slot, int rel) {
     constexpr bool exact = decltype(exact_c)::value;
     const bool masked = (j == static_cast<uint32_t>(K));
-    mbar_wait(&S.full, phase);
+    mbar_wait_spin(&S.full, phase);
     phase ^= 1u;
 
     // ---- shared -> registers: chunk i of this thread is float4 number GT*i + tg (conflict-free 128-bit
@@ -863,19 +835,13 @@ inline bool stream_kernel_supports(const StepParams& p) {
 }
 
 // every group must be able to queue all of its rows for rescoring (RC * NG = 8192 rows per CTA in every shape)
-inline long long stream_kernel_max_rows() {
-  int dev = 0, sms = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  return 8192LL * sms;
-}
+inline long long stream_kernel_max_rows() { return 8192LL * host::sm_count(); }
 
 template <int NP, int CPT, bool HAS_U, bool RECON, int LD>
 int launch_step_stream_r(const StepParams& p, cudaStream_t s) {
   using Sh = StreamShape<NP, CPT, HAS_U>;
-  int dev = 0, sms = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return D3PM_ERR_CUDA;
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return D3PM_ERR_CUDA;
+  const int sms = host::sm_count();
+  if (sms == 0) return D3PM_ERR_CUDA;
   const size_t smem = sizeof(GroupSmem<NP, CPT, HAS_U>) * Sh::NG + kCoefSmemRows * 16 * sizeof(float);
   auto kern = step_stream_kernel<NP, CPT, HAS_U, RECON, LD>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)) != cudaSuccess)
