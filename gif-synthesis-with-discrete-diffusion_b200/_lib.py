@@ -62,7 +62,7 @@ class TrainDesc(ctypes.Structure):
         ("B", c_int32), ("N", c_int32), ("K", c_int32), ("T", c_int32),
         ("pitch", c_int64), ("pitch_grad", c_int64),
         ("mask_weight_masked", c_float), ("mask_weight_unmasked", c_float),
-        ("backward", c_int32), ("stream", c_void_p),
+        ("backward", c_int32), ("stream", c_void_p), ("logits_dtype", c_int32),
     ]
 
 

@@ -298,16 +298,19 @@ int d3pm_train_rows(const d3pm_train_desc* d) {
     return fail(D3PM_ERR_INVALID, "train_rows: logits, x0, x_t, t and coef_table are required");
   if (d->B <= 0 || d->N <= 0 || d->K <= 0 || d->T <= 0) return fail(D3PM_ERR_INVALID, "train_rows: sizes must be positive");
   if (d->K % 4 != 0 || d->K > 8192) return fail(D3PM_ERR_UNSUPPORTED, "train_rows: K=%d must be a multiple of 4 and <= 8192", d->K);
-  if (d->pitch < d->K || d->pitch % 4 != 0 || !aligned16(d->logits) || !aligned16(d->coef_table))
-    return fail(D3PM_ERR_ALIGN, "train_rows: logits rows need pitch >= K, pitch %% 4 == 0, 16-byte base");
+  if (d->logits_dtype < D3PM_LOGITS_F32 || d->logits_dtype > D3PM_LOGITS_BF16)
+    return fail(D3PM_ERR_INVALID, "train_rows: unknown logits_dtype %d", d->logits_dtype);
+  const int pitch_mult = d->logits_dtype == D3PM_LOGITS_F32 ? 4 : 8;  // rows start on 16-byte boundaries
+  if (d->pitch < d->K || d->pitch % pitch_mult != 0 || !aligned16(d->logits) || !aligned16(d->coef_table))
+    return fail(D3PM_ERR_ALIGN, "train_rows: logits rows need pitch >= K, pitch %% %d == 0, 16-byte base", pitch_mult);
   const int64_t rows = static_cast<int64_t>(d->B) * d->N;
   if (rows > kMaxGrid) return fail(D3PM_ERR_UNSUPPORTED, "train_rows: B*N too large");
   if (d->backward < 0 || d->backward > 2) return fail(D3PM_ERR_INVALID, "train_rows: backward must be 0, 1 or 2");
   if (d->backward != 0) {
     if (d->grad == nullptr || d->w_main == nullptr || d->w_aux == nullptr)
       return fail(D3PM_ERR_INVALID, "train_rows: the gradient needs grad, w_main and w_aux");
-    if (d->pitch_grad < d->K || d->pitch_grad % 4 != 0 || !aligned16(d->grad))
-      return fail(D3PM_ERR_ALIGN, "train_rows: grad rows need pitch >= K, pitch %% 4 == 0, 16-byte base");
+    if (d->pitch_grad < d->K || d->pitch_grad % pitch_mult != 0 || !aligned16(d->grad))
+      return fail(D3PM_ERR_ALIGN, "train_rows: grad rows need pitch >= K, pitch %% %d == 0, 16-byte base", pitch_mult);
   }
   if (d->backward != 1 && (d->tok_main == nullptr || d->tok_aux == nullptr))
     return fail(D3PM_ERR_INVALID, "train_rows: the forward outputs need tok_main and tok_aux");
@@ -318,8 +321,14 @@ int d3pm_train_rows(const d3pm_train_desc* d) {
   p.B = d->B, p.N = d->N, p.K = d->K, p.T = d->T, p.pitch = d->pitch, p.pitch_grad = d->pitch_grad;
   p.mask_weight_masked = d->mask_weight_masked, p.mask_weight_unmasked = d->mask_weight_unmasked;
   p.rows = rows;
+  p.logits_dtype = d->logits_dtype;
+  if (d->backward == 0) p.grad = nullptr;  // a forward pass writes no gradient: its pitch does not matter
   const cudaStream_t s = static_cast<cudaStream_t>(d->stream);
-  if (d3pm::train_stream_supports(p) && (d->x0_recon == nullptr) == (d->xtm1_recon == nullptr)) {
+  const bool can_stream = d3pm::train_stream_supports(p) && (d->x0_recon == nullptr) == (d->xtm1_recon == nullptr);
+  if (d->logits_dtype != D3PM_LOGITS_F32 && !can_stream)
+    return fail(D3PM_ERR_UNSUPPORTED, "train_rows: 16-bit logits are read by the stream kernel only (K in {1024,2048,4096}, "
+                                      ">= 2048 rows, both or neither of x0_recon / xtm1_recon); cast to float for other shapes");
+  if (can_stream) {
     if (d->backward == 1) p.tok_main = nullptr, p.tok_aux = nullptr, p.x0_recon = nullptr, p.xtm1_recon = nullptr;
     const int rc = d3pm::launch_train_stream(p, d->backward != 0, s);
     if (rc != D3PM_OK) return fail(rc, "train_rows: stream kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));

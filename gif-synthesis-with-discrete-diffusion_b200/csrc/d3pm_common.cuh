@@ -74,6 +74,10 @@ __device__ __forceinline__ void st_stream4(float* p, float4 v) {
   asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
                : "memory");
 }
+// the 64-bit counterpart, for four 16-bit values
+__device__ __forceinline__ void st_stream_b64(void* p, uint32_t lo, uint32_t hi) {
+  asm volatile("st.global.cs.v2.b32 [%0], {%1,%2};" ::"l"(p), "r"(lo), "r"(hi) : "memory");
+}
 
 __device__ __forceinline__ float warp_max(float x) {
   float m;  // CREDUX.MAX.F32 on sm_100a: one instruction instead of five shuffles

@@ -28,6 +28,7 @@
 // HBM traffic is the algorithmic minimum: each logit is read once, 8 bytes of token go out per row.
 #pragma once
 
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include <type_traits>
@@ -139,6 +140,33 @@ struct LogitType {
   }
   static __device__ __forceinline__ const void* row(const float* base, unsigned long long elements) {
     return reinterpret_cast<const unsigned char*>(base) + elements * kBytes;
+  }
+  // Rows written in the logits' type (the training kernel's gradient): fp32 values narrowed with round-to-nearest-even,
+  // which is what `tensor.to(torch.float16 / torch.bfloat16)` does, so a 16-bit row equals the fp32 row cast afterwards.
+  using Elem = std::conditional_t<LD == D3PM_LOGITS_F32, float, unsigned short>;
+  static __device__ __forceinline__ uint32_t narrow2(float lo, float hi) {
+    uint32_t bits;
+    if constexpr (LD == D3PM_LOGITS_BF16) {
+      const __nv_bfloat162 v = __float22bfloat162_rn(make_float2(lo, hi));
+      bits = *reinterpret_cast<const uint32_t*>(&v);
+    } else {
+      const __half2 v = __float22half2_rn(make_float2(lo, hi));
+      bits = *reinterpret_cast<const uint32_t*>(&v);
+    }
+    return bits;
+  }
+  static __device__ __forceinline__ Elem narrow1(float v) {
+    if constexpr (LD == D3PM_LOGITS_F32) return v;
+    else if constexpr (LD == D3PM_LOGITS_BF16) return __bfloat16_as_ushort(__float2bfloat16_rn(v));
+    else return __half_as_ushort(__float2half_rn(v));
+  }
+  // classes 4q .. 4q+3 of an output row, one streaming store (16 bytes for fp32, 8 for the 16-bit types)
+  static __device__ __forceinline__ void store4(Elem* rowp, uint32_t q, const float (&o)[4]) {
+    if constexpr (LD == D3PM_LOGITS_F32) {
+      st_stream4(rowp + 4 * q, make_float4(o[0], o[1], o[2], o[3]));
+    } else {
+      st_stream_b64(rowp + 4 * q, narrow2(o[0], o[1]), narrow2(o[2], o[3]));
+    }
   }
 };
 // the NW per-warp values of a reduction, read back in one shared-memory load (unused lanes of the float4 = neutral)

@@ -39,6 +39,7 @@ struct TrainParams {
   int64_t pitch, pitch_grad;
   float mask_weight_masked, mask_weight_unmasked;
   int64_t rows;
+  int32_t logits_dtype;    // D3PM_LOGITS_*: element type of the logits and grad rows (16-bit: stream kernel only)
 };
 
 template <int NW>

@@ -11,6 +11,9 @@
 //   * the sum over classes of the gradient's softmax term is obtained in closed form from sums accumulated in the
 //     forward sweep, so a row needs two group exchanges (none across warps for the one-warp groups), not four;
 //   * the gradient row is written with streaming 128-bit stores straight from registers;
+//   * float16 / bfloat16 logits (LD, a denoiser run under autocast) are copied as they lie in HBM and widened in registers
+//     (LogitType, as in the reverse step); the gradient row then has the logits' type, each fp32 value rounded to nearest
+//     even - bit-identical to the fp32 kernel on logits.float() followed by grad.to(dtype), at half the bytes each way;
 //   * a row's scalars (x_0, x_t, t of its video, the per-video gradient weights) are loaded one row ahead and the
 //     coefficient table is staged in shared memory.
 // HBM traffic is the algorithmic minimum of a fused forward + backward: 16 KiB read and 16 KiB written per token.
@@ -46,26 +49,29 @@ struct TrainShape {
   static constexpr int NG = THREADS / GT;         // groups per CTA: 4 / 8 / 16
 };
 
-template <int NP>
+template <int NP, int LD = D3PM_LOGITS_F32>
 struct __align__(128) TrainGroupSmem {
-  float stage[2][1024 * NP];           // two rows per group in flight while a third is processed from registers
+  // two rows per group in flight while a third is processed from registers (16-bit rows: half the bytes)
+  float stage[2][1024 * NP * LogitType<LD>::kBytes / sizeof(float)];
   alignas(16) float red[2][4 * 4];     // reduction scratch: [value][warp], padded to four warps
   unsigned long long keys[2][4];
   unsigned long long full[2];
 };
 
-// WRITE_GRAD false: forward only (per-token losses, arg-maxes); true: forward + gradient rows in the same pass
-template <int NP, bool WRITE_GRAD>
+// WRITE_GRAD false: forward only (per-token losses, arg-maxes); true: forward + gradient rows in the same pass.
+// LD: D3PM_LOGITS_* of the logits and gradient rows.
+template <int NP, bool WRITE_GRAD, int LD = D3PM_LOGITS_F32>
 __global__ void __launch_bounds__(TrainShape<NP>::THREADS, 1) train_stream_kernel(const TrainParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   using Sh = TrainShape<NP>;
+  using LT = LogitType<LD>;
   constexpr int K = Sh::K, NC = Sh::CPT, GT = Sh::GT, NW = Sh::NW, NG = Sh::NG;
-  constexpr uint32_t kRowBytes = K * sizeof(float);
+  constexpr uint32_t kRowBytes = K * LT::kBytes;
   uint32_t tid;
   asm volatile("mov.u32 %0, %%tid.x;" : "=r"(tid));
   const int g = tid / GT, tg = tid % GT;
   const int lane = tid & 31, warp = (tid >> 5) & (NW - 1);
-  TrainGroupSmem<NP>& S = reinterpret_cast<TrainGroupSmem<NP>*>(smem_raw)[g];
+  TrainGroupSmem<NP, LD>& S = reinterpret_cast<TrainGroupSmem<NP, LD>*>(smem_raw)[g];
   const StreamSync<NW> sync{g + 1};
   // row indices are 32-bit (the launcher refuses more than 2^31 - 1 rows)
   const int G = static_cast<int>(gridDim.x) * NG;
@@ -74,7 +80,7 @@ __global__ void __launch_bounds__(TrainShape<NP>::THREADS, 1) train_stream_kerne
   auto issue_row = [&](int row, int st) {
     fence_proxy_async();
     mbar_expect_tx(&S.full[st], kRowBytes);
-    tma_load(S.stage[st], p.logits + static_cast<long long>(row) * p.pitch, kRowBytes, &S.full[st]);
+    tma_load(S.stage[st], LT::row(p.logits, static_cast<unsigned long long>(row) * p.pitch), kRowBytes, &S.full[st]);
   };
   if (tg == 0) {
     // A fence after each init, as the kernel was tuned.  One fence after both changes the machine code only in this
@@ -85,7 +91,7 @@ __global__ void __launch_bounds__(TrainShape<NP>::THREADS, 1) train_stream_kerne
     fence_mbarrier_init();
   }
   // CTA-wide copy of the coefficient table (16 floats per timestep) when it fits
-  float* coef_s = reinterpret_cast<float*>(smem_raw + sizeof(TrainGroupSmem<NP>) * NG);
+  float* coef_s = reinterpret_cast<float*>(smem_raw + sizeof(TrainGroupSmem<NP, LD>) * NG);
   const bool coef_in_smem = p.T <= kCoefSmemRows;
   if (coef_in_smem) {
     for (int i = tid; i < p.T * 16; i += Sh::THREADS)
@@ -136,11 +142,8 @@ __global__ void __launch_bounds__(TrainShape<NP>::THREADS, 1) train_stream_kerne
     // the first sweep on their softmax numerators (in place)
     float2 e[NC][2];
 #pragma unroll
-    for (int i = 0; i < NC; ++i) {
-      const float4 a = lds4(rowbuf + 4 * (GT * i + tg));
-      e[i][0] = make_float2(a.x, a.y), e[i][1] = make_float2(a.z, a.w);
-    }
-    const float c_x0 = rowbuf[x0], c_j = masked ? 0.f : rowbuf[j];
+    for (int i = 0; i < NC; ++i) LT::chunk(rowbuf, GT * i + tg, e[i][0], e[i][1]);
+    const float c_x0 = LT::one(rowbuf, x0), c_j = masked ? 0.f : LT::one(rowbuf, j);
 
     // ---- exchange 1: (max, sum of exponentials relative to the thread-local max) and the arg-max of the logits ----
     float m = fmaxf(fmaxf(e[0][0].x, e[0][0].y), fmaxf(e[0][1].x, e[0][1].y));
@@ -432,7 +435,7 @@ __global__ void __launch_bounds__(TrainShape<NP>::THREADS, 1) train_stream_kerne
     const float h_j = open_j ? p_j * fmaf(gP_j, cf.AS, cf.WS * Gs) : 0.f;
     const float gA = g_gen * cf.A, WG = cf.W * Gs;
     const float hsum = fmaf(gA, sPP - gpp_x0 - gpp_j, WG * (sP - gpo_x0 - gpo_j)) + h_x0 + h_j;
-    float* __restrict__ rg = p.grad + static_cast<long long>(row) * p.pitch_grad;
+    typename LT::Elem* __restrict__ rg = reinterpret_cast<typename LT::Elem*>(p.grad) + static_cast<long long>(row) * p.pitch_grad;
     const uint32_t q_x0 = x0 >> 2, q_j = j_other ? (j >> 2) : 0xffffffffu;
 #pragma unroll
     for (int i = 0; i < NC; ++i) {
@@ -454,11 +457,11 @@ __global__ void __launch_bounds__(TrainShape<NP>::THREADS, 1) train_stream_kerne
           o[c] = fminf(sm, 1.0f) * hk - sm * hsum;
         }
       }
-      st_stream4(rg + 4 * q, make_float4(o[0], o[1], o[2], o[3]));
+      LT::store4(rg, q, o);
     }
     // the two special classes: their owners overwrite the generic value (same thread, same address: program order)
-    if (tg == static_cast<int>(q_x0 & static_cast<uint32_t>(GT - 1))) rg[x0] = fmaf(-sm_x0, hsum, h_x0);
-    if (j_other && tg == static_cast<int>(q_j & static_cast<uint32_t>(GT - 1))) rg[j] = fmaf(-sm_j, hsum, h_j);
+    if (tg == static_cast<int>(q_x0 & static_cast<uint32_t>(GT - 1))) rg[x0] = LT::narrow1(fmaf(-sm_x0, hsum, h_x0));
+    if (j_other && tg == static_cast<int>(q_j & static_cast<uint32_t>(GT - 1))) rg[j] = LT::narrow1(fmaf(-sm_j, hsum, h_j));
   }
   if (status_bits != 0 && tg == 0 && p.status != nullptr) atomicOr(p.status, status_bits);
 }
@@ -478,28 +481,40 @@ __global__ void __launch_bounds__(256) scale_rows_kernel(float* __restrict__ row
   }
 }
 
+// 16-bit rows start on 16-byte boundaries too: both pitches a multiple of 8 elements
 inline bool train_stream_supports(const TrainParams& p) {
-  return (p.K == 1024 || p.K == 2048 || p.K == 4096) && p.rows >= 2048 && p.pitch % 4 == 0;
+  return (p.K == 1024 || p.K == 2048 || p.K == 4096) && p.rows >= 2048 && p.pitch % 4 == 0 &&
+         (p.logits_dtype == D3PM_LOGITS_F32 || (p.pitch % 8 == 0 && (p.grad == nullptr || p.pitch_grad % 8 == 0)));
 }
 
-template <int NP, bool WRITE_GRAD>
+template <int NP, bool WRITE_GRAD, int LD>
 int launch_train_stream_t(const TrainParams& p, cudaStream_t s) {
   const int sms = host::sm_count();
   if (sms == 0) return D3PM_ERR_CUDA;
-  const size_t smem = sizeof(TrainGroupSmem<NP>) * TrainShape<NP>::NG + kCoefSmemRows * 16 * sizeof(float);
-  auto kern = train_stream_kernel<NP, WRITE_GRAD>;
+  const size_t smem = sizeof(TrainGroupSmem<NP, LD>) * TrainShape<NP>::NG + kCoefSmemRows * 16 * sizeof(float);
+  auto kern = train_stream_kernel<NP, WRITE_GRAD, LD>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)) != cudaSuccess)
     return D3PM_ERR_CUDA;
   kern<<<static_cast<unsigned>(sms), TrainShape<NP>::THREADS, smem, s>>>(p);
   return D3PM_OK;
 }
 
-inline int launch_train_stream(const TrainParams& p, bool write_grad, cudaStream_t s) {
+template <int LD>
+int launch_train_stream_ld(const TrainParams& p, bool write_grad, cudaStream_t s) {
   switch (p.K) {
-    case 1024: return write_grad ? launch_train_stream_t<1, true>(p, s) : launch_train_stream_t<1, false>(p, s);
-    case 2048: return write_grad ? launch_train_stream_t<2, true>(p, s) : launch_train_stream_t<2, false>(p, s);
-    case 4096: return write_grad ? launch_train_stream_t<4, true>(p, s) : launch_train_stream_t<4, false>(p, s);
+    case 1024: return write_grad ? launch_train_stream_t<1, true, LD>(p, s) : launch_train_stream_t<1, false, LD>(p, s);
+    case 2048: return write_grad ? launch_train_stream_t<2, true, LD>(p, s) : launch_train_stream_t<2, false, LD>(p, s);
+    case 4096: return write_grad ? launch_train_stream_t<4, true, LD>(p, s) : launch_train_stream_t<4, false, LD>(p, s);
     default: return D3PM_ERR_UNSUPPORTED;
+  }
+}
+
+inline int launch_train_stream(const TrainParams& p, bool write_grad, cudaStream_t s) {
+  switch (p.logits_dtype) {
+    case D3PM_LOGITS_F32: return launch_train_stream_ld<D3PM_LOGITS_F32>(p, write_grad, s);
+    case D3PM_LOGITS_F16: return launch_train_stream_ld<D3PM_LOGITS_F16>(p, write_grad, s);
+    case D3PM_LOGITS_BF16: return launch_train_stream_ld<D3PM_LOGITS_BF16>(p, write_grad, s);
+    default: return D3PM_ERR_INVALID;
   }
 }
 

@@ -645,7 +645,8 @@ class FusedDiffusionTransformer(nn.Module):
         else:
             out = self.transformer(xt, cond_emb, t)
         assert out.size(0) == xt.size(0) and out.size(1) == self.num_classes - 1 and out.size()[2:] == xt.size()[1:]
-        out = out.float()
+        if out.dtype not in (torch.float16, torch.bfloat16):
+            out = out.float()  # 16-bit logits (autocast) go to the loss kernel as they are; their gradient comes back 16-bit
 
         aux_on = self.auxiliary_loss_weight != 0 and is_train
         if aux_on:
@@ -677,7 +678,7 @@ class FusedDiffusionTransformer(nn.Module):
         log_model_prob = None
         if need_log_model_prob:
             with torch.no_grad():
-                rows, _ = train._logit_rows(out.detach())
+                rows, _ = train._logit_rows(out.detach().float())  # the row kernel that writes `post` reads fp32
                 post = ops.fused_step(rows, None, xt, t.contiguous(), self.coef_table(), guidance_scale=1.0,
                                       sample_mode=_lib.SAMPLE_NONE, want_post=True, status=self._status_word())["post"]
                 log_model_prob = ops.as_logical(post, self.num_classes)

@@ -188,7 +188,7 @@ int d3pm_q_sample_tokens(const int64_t* x0, const int64_t* t, const float* sched
  *                  upstream gradient later rescales per video with d3pm_scale_rows (free when the factor is 1).
  * K in {1024, 2048, 4096} with >= 2048 rows runs the persistent TMA-pipelined kernel, other shapes one CTA per row.  */
 typedef struct d3pm_train_desc {
-  const float* logits;   /* [B*N][pitch] denoiser logits (first K valid) */
+  const float* logits;   /* [B*N][pitch] denoiser logits (first K valid); element type = logits_dtype */
   const int64_t* x0;     /* [B*N] in [0, K) */
   const int64_t* x_t;    /* [B*N] in [0, K] */
   const int64_t* t;      /* [B] */
@@ -199,13 +199,19 @@ typedef struct d3pm_train_desc {
   float* tok_aux;        /* [B*N], forward only */
   int64_t* x0_recon;     /* [B*N] arg-max of p(x0 | x_t), nullable (forward) */
   int64_t* xtm1_recon;   /* [B*N] arg-max of the model posterior, nullable (forward) */
-  float* grad;           /* [B*N][pitch_grad], backward only */
+  float* grad;           /* [B*N][pitch_grad], backward only; element type = logits_dtype */
   uint32_t* status;
   int32_t B, N, K, T;
-  int64_t pitch, pitch_grad;
+  int64_t pitch, pitch_grad; /* in elements of logits_dtype */
   float mask_weight_masked, mask_weight_unmasked; /* mask_weight[0], mask_weight[1] (:423) */
   int32_t backward;
   d3pm_stream_t stream;
+  int32_t logits_dtype;  /* D3PM_LOGITS_* of the logits AND grad rows (0 = F32).  16-bit logits are read as they lie in HBM and
+                            widened in registers; the gradient is computed in fp32 and written in the same 16-bit type, rounded
+                            to nearest even - bit-identical to running the fp32 path on logits.float() and casting grad with
+                            tensor.to(dtype), at half the traffic each way.  Stream kernel only (K in {1024,2048,4096}, >= 2048
+                            rows, both or neither of x0_recon / xtm1_recon; pitch and pitch_grad % 8 == 0, else
+                            D3PM_ERR_ALIGN); other shapes return D3PM_ERR_UNSUPPORTED and the caller casts */
 } d3pm_train_desc;
 
 int d3pm_train_rows(const d3pm_train_desc* desc);

@@ -1,6 +1,6 @@
-"""Compare the machine code of two builds of libd3pm_b200.so, kernel by kernel.
+r"""Compare the machine code of two builds of libd3pm_b200.so, kernel by kernel.
 
-    python tools/sass_compare.py OLD.so NEW.so [--context 3]
+    python tools/sass_compare.py OLD.so NEW.so [--context 3] [--rename PATTERN=REPLACEMENT ...]
 
 Runs `cuobjdump -sass` on both libraries, splits each listing at its `Function :` lines and compares the kernels by
 mangled name.  Reports the kernels that exist in only one build, the number that are byte-identical, and for each kernel
@@ -8,6 +8,9 @@ that differs a diff of its instructions, plus whether every change lies in the k
 CTA-wide barrier (`__syncthreads()`, BAR.SYNC 0x0).  In that diff the encodings are dropped and the code addresses
 inside instructions (branch targets, return addresses) are rewritten relative to the instruction, so code that merely
 moved after an inserted or removed instruction compares equal.  Addresses shown are those of NEW.so.
+--rename applies a regular-expression substitution to the kernel names of OLD.so before they are matched, for a kernel
+whose mangled name changed while its code should not, e.g. a template that gained a parameter with a default value
+(`--rename 'train_stream_kernelILi(\d)ELb(\d)EE=train_stream_kernelILi\1ELb\2ELi0EE'`).
 Exit status 0 when every kernel is present in both builds and identical, 1 otherwise.
 """
 import argparse
@@ -80,8 +83,13 @@ def main():
     ap.add_argument("old")
     ap.add_argument("new")
     ap.add_argument("--context", type=int, default=3, help="unchanged instructions shown around each change")
+    ap.add_argument("--rename", action="append", default=[], metavar="PATTERN=REPLACEMENT",
+                    help="re.sub applied to the kernel names of OLD before matching (repeatable)")
     a = ap.parse_args()
     old, new = functions(a.old), functions(a.new)
+    for rule in a.rename:
+        pattern, _, replacement = rule.partition("=")
+        old = {re.sub(pattern, replacement, name): text for name, text in old.items()}
     only_old, only_new = sorted(set(old) - set(new)), sorted(set(new) - set(old))
     common = sorted(set(old) & set(new))
     differ = [f for f in common if old[f] != new[f]]

@@ -2,7 +2,12 @@
 4096 codes.  Times `d3pm_train_rows` forward and backward (CUDA events) and, with --cpu, the oracle port of the
 reference's `_train_loss` + autograd backward on the host cores.
 
-    python tools/train_bench.py [--videos 16] [--tokens 1024] [--cpu]
+With --dtype float16 | bfloat16 it compares, at --videos and at 64 videos, the two ways to train on 16-bit logits:
+(a) the losses (backward = 0) and then the gradient (backward = 1) straight on the 16-bit rows, and (b) the cast route:
+`.float()`, the fp32 one-pass kernel (backward = 2), `grad.to(dtype)`, and the same with a `d3pm_scale_rows` factor
+other than 1 (any run with a loss scaler).  The routes alternate in one process, CUDA events, median of the rounds.
+
+    python tools/train_bench.py [--videos 16] [--tokens 1024] [--cpu] [--dtype float16|bfloat16]
 """
 import argparse
 import os
@@ -20,6 +25,8 @@ ap.add_argument("--videos", type=int, default=16)
 ap.add_argument("--tokens", type=int, default=1024)
 ap.add_argument("--codes", type=int, default=4096)
 ap.add_argument("--cpu", action="store_true")
+ap.add_argument("--dtype", choices=("float16", "bfloat16"), help="compare the 16-bit route with the cast route")
+ap.add_argument("--rounds", type=int, default=7, help="alternated rounds of the --dtype comparison")
 a = ap.parse_args()
 B, N, K, T = a.videos, a.tokens, a.codes, 100
 dev = torch.device("cuda", 0)
@@ -54,6 +61,56 @@ def bwd():
 def both():
     return train._train_rows(logits, K, x0, x_t, t, table, (1, 1), backward=2, w_main=w, w_aux=w, want_recon=True)
 
+
+
+
+def compare_16bit(B, dtype, rounds, iters=10):
+    """Times the 16-bit route against the cast route on the same [B, N, K] logits (inputs >> L2 at 64 videos)."""
+    gen = torch.Generator(device=dev).manual_seed(1)
+    l16 = torch.randn(B, N, K, device=dev, generator=gen).to(dtype)
+    xs = torch.randint(0, K, (B, N), device=dev, generator=gen)
+    ts = torch.randint(0, T, (B,), device=dev, generator=gen)
+    xts = m.q_sample_tokens(xs, ts)
+    ones, half = torch.ones(B, device=dev), torch.full((B,), 0.5, device=dev)
+
+    def new():
+        train._train_rows(l16, K, xs, xts, ts, table, (1, 1), backward=0, want_recon=True)
+        return train._train_rows(l16, K, xs, xts, ts, table, (1, 1), backward=1, w_main=ones, w_aux=ones)["grad"]
+
+    def cast(factor=None):
+        out = train._train_rows(l16.float(), K, xs, xts, ts, table, (1, 1), backward=2, w_main=ones, w_aux=ones,
+                                want_recon=True)
+        if factor is not None:
+            train.scale_rows(out["grad"], factor)
+        return out["grad"].to(dtype)
+
+    e = B * N * K  # bytes per route: the logits' and the gradient's reads and writes, 2 bytes per 16-bit, 4 per fp32 value
+    routes = (("16-bit rows: losses, then gradient", new, e * (2 + 2 + 2)),
+              ("cast route: .float(), one fp32 pass, .to(dtype)", cast, e * (2 + 4 + 4 + 4 + 4 + 2)),
+              ("cast route with a loss-scale rescale", lambda: cast(half), e * (2 + 4 + 4 + 4 + 4 + 4 + 4 + 2)))
+    for _, fn, _ in routes:
+        fn()
+    times = {name: [] for name, _, _ in routes}
+    for _ in range(rounds):
+        for name, fn, _ in routes:
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(iters):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            times[name].append(e0.elapsed_time(e1) / iters)
+    for name, _, nbytes in routes:
+        ms = sorted(times[name])[len(times[name]) // 2]
+        print(f"{dtype} {B}x{N} tokens x {K} codes, {name}: {ms:.3f} ms (median of {rounds}, spread "
+              f"{min(times[name]):.3f}-{max(times[name]):.3f}), {nbytes / 1e9:.3f} GB algorithmic, {nbytes / ms / 1e6:.0f} GB/s")
+
+
+if a.dtype:
+    print(torch.cuda.get_device_name(dev))
+    for videos in sorted({B, 64}):
+        compare_16bit(videos, getattr(torch, a.dtype), a.rounds)
+    sys.exit(0)
 
 for name, fn, nbytes in (("forward (losses, arg-maxes)", fwd, B * N * K * 4), ("gradient only", bwd, 2 * B * N * K * 4),
                          ("forward + gradient, one pass", both, 2 * B * N * K * 4)):
