@@ -4,6 +4,7 @@
 // the file, which owns device staging buffers and two streams for callers whose inputs are HOST buffers.
 #include <cstdarg>
 #include <cstdio>
+#include <type_traits>
 
 #include "d3pm_host.h"
 #include "d3pm_ops.cuh"
@@ -57,16 +58,21 @@ void launch_rows(const d3pm::StepParams& p, cudaStream_t s) {
 }
 
 template <int V>
-void launch_rows_u(const d3pm::StepParams& p, cudaStream_t s) {
-  if (p.logits_u != nullptr) launch_rows<V, true>(p, s);
-  else launch_rows<V, false>(p, s);
-}
-
-template <int V>
 void launch_train(const d3pm::TrainParams& p, bool backward, cudaStream_t s) {
   const dim3 grid(static_cast<unsigned>(p.rows)), block(d3pm::kRowThreads);
   if (backward) d3pm::train_rows_kernel<V, true><<<grid, block, 0, s>>>(p);
   else d3pm::train_rows_kernel<V, false><<<grid, block, 0, s>>>(p);
+}
+
+// launch(std::integral_constant<int, V>) with V = float4 chunks per thread of a one-CTA-per-row kernel: the fewest of
+// 1, 2, 4, 8 that cover K classes
+template <typename Launch>
+void with_row_chunks(int K, Launch launch) {
+  const int chunks = (K / 4 + d3pm::kRowThreads - 1) / d3pm::kRowThreads;
+  if (chunks <= 1) launch(std::integral_constant<int, 1>{});
+  else if (chunks <= 2) launch(std::integral_constant<int, 2>{});
+  else if (chunks <= 4) launch(std::integral_constant<int, 4>{});
+  else launch(std::integral_constant<int, 8>{});
 }
 
 }  // namespace
@@ -162,11 +168,10 @@ int d3pm_fused_step(const d3pm_step_desc* d) {
     if (rc != D3PM_OK) return fail(rc, "fused_step: stream kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     return check_launch("fused_step(stream)");
   }
-  const int chunks = (d->K / 4 + d3pm::kRowThreads - 1) / d3pm::kRowThreads;
-  if (chunks <= 1) launch_rows_u<1>(p, s);
-  else if (chunks <= 2) launch_rows_u<2>(p, s);
-  else if (chunks <= 4) launch_rows_u<4>(p, s);
-  else launch_rows_u<8>(p, s);
+  with_row_chunks(d->K, [&](auto v) {
+    if (p.logits_u != nullptr) launch_rows<decltype(v)::value, true>(p, s);
+    else launch_rows<decltype(v)::value, false>(p, s);
+  });
   return check_launch("fused_step");
 }
 
@@ -334,14 +339,10 @@ int d3pm_train_rows(const d3pm_train_desc* d) {
     if (rc != D3PM_OK) return fail(rc, "train_rows: stream kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     return check_launch("train_rows(stream)");
   }
-  const int chunks = (d->K / 4 + d3pm::kRowThreads - 1) / d3pm::kRowThreads;
   for (int pass = 0; pass < 2; ++pass) {  // one CTA per row: forward and gradient are separate launches
     const bool bwd = pass == 1;
     if ((bwd && d->backward == 0) || (!bwd && d->backward == 1)) continue;
-    if (chunks <= 1) launch_train<1>(p, bwd, s);
-    else if (chunks <= 2) launch_train<2>(p, bwd, s);
-    else if (chunks <= 4) launch_train<4>(p, bwd, s);
-    else launch_train<8>(p, bwd, s);
+    with_row_chunks(d->K, [&](auto v) { launch_train<decltype(v)::value>(p, bwd, s); });
   }
   return check_launch("train_rows");
 }

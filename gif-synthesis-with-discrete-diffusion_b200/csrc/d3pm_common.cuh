@@ -1,4 +1,4 @@
-// Shared device helpers for the D3PM reverse-step kernels (sm_100a only).
+// Shared device helpers for the D3PM reverse-step and training kernels (sm_100a only).
 //
 // Math notation follows DESIGN.md §3 / SURVEY.md §8(a8).  Reference lines are those of
 // src/models/motionencoder/diffusion_transformer.py.
@@ -56,6 +56,15 @@ __device__ __forceinline__ float lg2(float x) {
   float y;
   asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
+}
+// exact residual of the fp32 product m*log2e (natural-log units -> log2 units)
+__device__ __forceinline__ float to_log2_units(float m) { return __fmul_rn(m, kLog2e); }
+
+// ln(sum_k exp(x_k - M)) from S = sum_k 2^(x_k*log2e - fl(M*log2e)): corrects the rounding of M*log2e
+__device__ __forceinline__ float ln_rel_sum(float M, float S) {
+  const float m2 = to_log2_units(M);
+  const float delta = -fmaf(M, kLog2e, -m2);  // m2 - M*log2e, exact
+  return kLn2 * (lg2(S) + delta);
 }
 // clamp(log P, -70, 0): the single place the posterior leaves the linear domain, shared by every
 // sampling mode so that they agree bit for bit.
@@ -230,42 +239,13 @@ __device__ __forceinline__ float gumbel_from_uniform(float u) {
   return -logf(-logf(u + kTiny) + kTiny);
 }
 
+constexpr int kRowThreads = 256;  // threads of the one-CTA-per-row kernels (step_rows_kernel, train_rows_kernel)
+
 // ---- group reductions ------------------------------------------------------------------------
 // All threads of a group (NW warps) call these together; `sync` is the group's barrier.
 struct CtaSync {
   __device__ __forceinline__ void operator()() const { __syncthreads(); }
 };
-template <int ID, int THREADS>
-struct NamedSync {
-  __device__ __forceinline__ void operator()() const {
-    asm volatile("bar.sync %0, %1;" ::"n"(ID), "n"(THREADS) : "memory");
-  }
-};
-
-// Combine per-thread (max, sum of exp2(x*log2e - max*log2e)) pairs into the group's (max, sum).
-// m is in natural-log units (a raw logit); s is relative to m.  scratch: 2*NW floats.
-template <int NW, typename Sync>
-__device__ __forceinline__ void group_max_sum(float& m, float& s, float* scratch, Sync sync) {
-  const int lane = threadIdx.x & 31, warp = (threadIdx.x >> 5) % NW;
-  const float mw = warp_max(m);
-  const float sw = warp_sum(m == -CUDART_INF_F ? 0.0f : s * ex2((m - mw) * kLog2e));
-  if (lane == 0) {
-    scratch[warp] = mw;
-    scratch[NW + warp] = sw;
-  }
-  sync();
-  float M = scratch[0];
-#pragma unroll
-  for (int w = 1; w < NW; ++w) M = fmaxf(M, scratch[w]);
-  float S = 0.0f;
-#pragma unroll
-  for (int w = 0; w < NW; ++w) {
-    const float mwv = scratch[w];
-    S += (mwv == -CUDART_INF_F) ? 0.0f : scratch[NW + w] * ex2((mwv - M) * kLog2e);
-  }
-  m = M;
-  s = S;
-}
 
 template <int NW, typename Sync>
 __device__ __forceinline__ unsigned long long group_max_u64(unsigned long long key, unsigned long long* scratch,

@@ -39,16 +39,6 @@ struct StepParams {
   PhiloxRoundKeys keys;  // the round keys of `seed`, expanded on the host (stream kernel: constant-bank operands)
 };
 
-// exact residual of the fp32 product m*log2e (natural-log units -> log2 units)
-__device__ __forceinline__ float to_log2_units(float m) { return __fmul_rn(m, kLog2e); }
-
-// ln(sum_k exp(x_k - M)) from S = sum_k 2^(x_k*log2e - fl(M*log2e)): corrects the rounding of M*log2e
-__device__ __forceinline__ float ln_rel_sum(float M, float S) {
-  const float m2 = to_log2_units(M);
-  const float delta = -fmaf(M, kLog2e, -m2);  // m2 - M*log2e, exact
-  return kLn2 * (lg2(S) + delta);
-}
-
 // Everything a row needs once the softmax statistics are known.  Identical in every kernel.
 struct RowMath {
   float A, Bc;      // P_k = p_k*A + Bc           (k != x_t)
@@ -105,8 +95,6 @@ struct ThinRule {
     accept = -lg2(inv) * kLn2 + 0.02f;
   }
 };
-
-constexpr int kRowThreads = 256;
 
 template <int NV, int NW, typename Sync>
 __device__ __forceinline__ void group_max_sum_n(float (&m)[NV], float (&s)[NV], float* scratch, Sync sync) {

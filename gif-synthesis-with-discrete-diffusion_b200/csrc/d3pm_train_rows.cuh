@@ -17,7 +17,7 @@
 // pass recomputes the row and writes the gradient row: the logits are read once per pass, nothing else is stored.
 #pragma once
 
-#include "d3pm_step_rows.cuh"
+#include "d3pm_common.cuh"
 
 namespace d3pm {
 

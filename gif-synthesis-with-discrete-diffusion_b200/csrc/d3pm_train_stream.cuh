@@ -19,9 +19,8 @@
 // HBM traffic is the algorithmic minimum of a fused forward + backward: 16 KiB read and 16 KiB written per token.
 #pragma once
 
-#include "d3pm_host.h"
 #include "d3pm_ptx.cuh"
-#include "d3pm_step_stream.cuh"
+#include "d3pm_stream.cuh"
 #include "d3pm_train_rows.cuh"
 
 namespace d3pm {
@@ -487,24 +486,19 @@ inline bool train_stream_supports(const TrainParams& p) {
          (p.logits_dtype == D3PM_LOGITS_F32 || (p.pitch % 8 == 0 && (p.grad == nullptr || p.pitch_grad % 8 == 0)));
 }
 
-template <int NP, bool WRITE_GRAD, int LD>
-int launch_train_stream_t(const TrainParams& p, cudaStream_t s) {
-  const int sms = host::sm_count();
-  if (sms == 0) return D3PM_ERR_CUDA;
+template <int NP, int LD>
+int launch_train_stream_np(const TrainParams& p, bool write_grad, cudaStream_t s) {
   const size_t smem = sizeof(TrainGroupSmem<NP, LD>) * TrainShape<NP>::NG + kCoefSmemRows * 16 * sizeof(float);
-  auto kern = train_stream_kernel<NP, WRITE_GRAD, LD>;
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)) != cudaSuccess)
-    return D3PM_ERR_CUDA;
-  kern<<<static_cast<unsigned>(sms), TrainShape<NP>::THREADS, smem, s>>>(p);
-  return D3PM_OK;
+  return launch_persistent(write_grad ? train_stream_kernel<NP, true, LD> : train_stream_kernel<NP, false, LD>,
+                           TrainShape<NP>::THREADS, smem, p, s);
 }
 
 template <int LD>
 int launch_train_stream_ld(const TrainParams& p, bool write_grad, cudaStream_t s) {
   switch (p.K) {
-    case 1024: return write_grad ? launch_train_stream_t<1, true, LD>(p, s) : launch_train_stream_t<1, false, LD>(p, s);
-    case 2048: return write_grad ? launch_train_stream_t<2, true, LD>(p, s) : launch_train_stream_t<2, false, LD>(p, s);
-    case 4096: return write_grad ? launch_train_stream_t<4, true, LD>(p, s) : launch_train_stream_t<4, false, LD>(p, s);
+    case 1024: return launch_train_stream_np<1, LD>(p, write_grad, s);
+    case 2048: return launch_train_stream_np<2, LD>(p, write_grad, s);
+    case 4096: return launch_train_stream_np<4, LD>(p, write_grad, s);
     default: return D3PM_ERR_UNSUPPORTED;
   }
 }
