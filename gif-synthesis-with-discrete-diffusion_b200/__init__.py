@@ -7,7 +7,7 @@ log_sample_categorical / sample) on top of the C-ABI library `csrc/libd3pm_b200.
 (hand-written sm_100a CUDA, declared in `include/d3pm_b200.h`).  Import as `d3pm_b200`.
 """
 from d3pm_b200._lib import D3PMError, library_path, load_library  # noqa: F401
-from d3pm_b200 import decode, head, ops, train  # noqa: F401
+from d3pm_b200 import attention, decode, head, ops, train  # noqa: F401
 from d3pm_b200.diffusion_transformer import FusedDiffusionTransformer, alpha_schedule  # noqa: F401
 from d3pm_b200.distributed import gather_tokens, shard_range  # noqa: F401
 

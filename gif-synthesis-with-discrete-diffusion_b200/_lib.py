@@ -19,7 +19,7 @@ EXPORTED_SYMBOLS = (
     "d3pm_head_image_floats", "d3pm_head_prepare", "d3pm_head_step", "d3pm_scale_rows",
     "d3pm_decode_lut", "d3pm_tokens_to_features",
     "d3pm_dec_image_floats", "d3pm_dec_weight_image", "d3pm_dec_conv", "d3pm_dec_embed_rows", "d3pm_dec_axial_attention",
-    "d3pm_dec_col2im",
+    "d3pm_dec_col2im", "d3pm_self_attention",
     "d3pm_host_step_create", "d3pm_host_step_destroy", "d3pm_host_step_h2d_bytes", "d3pm_host_step_d2h_bytes",
     "d3pm_host_step_run", "d3pm_host_head_step_run", "d3pm_host_step_set_logits_dtype",
 )
@@ -93,6 +93,15 @@ class DecConvDesc(ctypes.Structure):
         ("relu_out", c_int32), ("terms", c_int32), ("n_tile", c_int32),
         ("tap", c_int8 * 4 * DEC_MAX_TAPS * DEC_MAX_CLASSES), ("cls", c_int8 * 4 * DEC_MAX_CLASSES),
         ("stream", c_void_p),
+    ]
+
+
+class AttnDesc(ctypes.Structure):
+    """Mirror of `d3pm_attn_desc`."""
+    _fields_ = [
+        ("q", c_void_p), ("k", c_void_p), ("v", c_void_p), ("y", c_void_p),
+        ("B", c_int32), ("N", c_int32), ("heads", c_int32), ("head_dim", c_int32),
+        ("pitch_qkv", c_int64), ("pitch_y", c_int64), ("scale", c_float), ("stream", c_void_p),
     ]
 
 
@@ -195,6 +204,8 @@ def load_library() -> ctypes.CDLL:
     lib.d3pm_dec_col2im.restype = c_int
     lib.d3pm_dec_col2im.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                     c_void_p]
+    lib.d3pm_self_attention.restype = c_int
+    lib.d3pm_self_attention.argtypes = [POINTER(AttnDesc)]
     lib.d3pm_to_token_major.restype = c_int
     lib.d3pm_to_token_major.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]
     _lib = lib

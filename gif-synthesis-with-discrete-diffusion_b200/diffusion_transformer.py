@@ -18,7 +18,7 @@ import numpy as np
 import torch
 from torch import nn
 
-from d3pm_b200 import _lib, head, ops, train
+from d3pm_b200 import _lib, attention, head, ops, train
 from d3pm_b200._lib import D3PMError
 
 _SCHEDULE_BUFFERS = ("log_at", "log_bt", "log_ct", "log_1_min_ct",
@@ -229,6 +229,15 @@ class FusedDiffusionTransformer(nn.Module):
                                 "(content_emb + blocks + to_logits, transformer_utils.py:429-444) or offer "
                                 "hidden_states(x_t, cond_emb, t) -> [B, N, n_embd], the input of its to_logits head")
         self.fuse_head = bool(enable)
+        return self
+
+    def enable_fused_attention(self, enable: bool = True):
+        """Run the self-attention of the denoiser's blocks (`FullAttention`, transformer_utils.py:24-62) on
+        `d3pm_self_attention`, which never forms the `[B, heads, N, N]` score matrix: `attention.fuse_self_attention` on
+        the denoiser (raises `D3PMError` if it has no FullAttention of head width 4).  Inference only - training,
+        autocast and masked calls still run the reference's module; `state_dict()` is unchanged.  Composes with
+        `enable_fused_head()` and the one-pass shared conditioning.  `enable=False` restores the original modules."""
+        attention.fuse_self_attention(self.transformer, enable)
         return self
 
     def _head_weights(self) -> "head.HeadWeights":

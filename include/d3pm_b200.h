@@ -348,6 +348,29 @@ int d3pm_dec_axial_attention(const float* qkv, float* att, int B, int T, int H, 
 int d3pm_dec_col2im(const float* y_t, const float* bias, float* out, int B, int T, int H, int W, int Cout, int st, int sh, int sw,
                     d3pm_stream_t stream);
 
+/* ---------------------------------------------------------------- denoiser self-attention (SURVEY.md §8 f3)
+ * The self-attention of the denoiser's blocks, FullAttention (transformer_utils.py:24-62), after its q / k / v Linears and
+ * before `proj`, forward only, fp32:
+ *     y[b*N + n][h*hd + c] = sum_j softmax_j(scale * q_{b,n,h} . k_{b,j,h}) v_{b,j,h}[c]
+ * with x_{b,n,h} = x[b*N + n][h*hd .. h*hd + hd).  q, k and v are rows of pitch_qkv floats as the three Linear outputs lie
+ * ([B*T][C] each, pitch_qkv = C); y is written as [B*N][pitch_y], the layout of the reference's
+ * `y.transpose(1, 2).contiguous().view(B, T, C)`.  The [N, N] scores never leave registers (no workspace), the softmax is
+ * exact (running maximum per block of 32 keys, ex2.approx on pre-scaled scores).  The head-averaged attention map the
+ * reference also returns is not produced.  head_dim = 4 (n_embd 64 / 16 heads, the shipped model) only: other values
+ * return D3PM_ERR_UNSUPPORTED.  Any N >= 1 and B >= 1, heads <= 65535; pointers 16-byte aligned, pitches % 4 == 0.       */
+typedef struct d3pm_attn_desc {
+  const float* q;      /* [B*N][pitch_qkv] */
+  const float* k;      /* [B*N][pitch_qkv] */
+  const float* v;      /* [B*N][pitch_qkv] */
+  float* y;            /* [B*N][pitch_y] out, columns [0, heads * head_dim) written */
+  int32_t B, N, heads, head_dim;
+  int64_t pitch_qkv, pitch_y; /* in floats, >= heads * head_dim */
+  float scale;         /* softmax scale, 1 / sqrt(head_dim) in the reference */
+  d3pm_stream_t stream;
+} d3pm_attn_desc;
+
+int d3pm_self_attention(const d3pm_attn_desc* desc);
+
 /* ---------------------------------------------------------------- host-buffer entry points
  * For a caller whose denoiser output lives in HOST memory (the reference's CPU tensors; bench.py's `e2e`): a handle owns
  * the device staging buffers for one batch shape, a copy stream and a compute stream.  `run` copies the inputs up in
