@@ -231,13 +231,18 @@ class FusedDiffusionTransformer(nn.Module):
         self.fuse_head = bool(enable)
         return self
 
-    def enable_fused_attention(self, enable: bool = True):
+    def enable_fused_attention(self, enable: bool = True, cross: bool = False):
         """Run the self-attention of the denoiser's blocks (`FullAttention`, transformer_utils.py:24-62) on
         `d3pm_self_attention`, which never forms the `[B, heads, N, N]` score matrix: `attention.fuse_self_attention` on
-        the denoiser (raises `D3PMError` if it has no FullAttention of head width 4).  Inference only - training,
-        autocast and masked calls still run the reference's module; `state_dict()` is unchanged.  Composes with
-        `enable_fused_head()` and the one-pass shared conditioning.  `enable=False` restores the original modules."""
+        the denoiser (raises `D3PMError` if it has no FullAttention of head width 4).  With `cross=True` the blocks'
+        cross-attention over the condition tokens (`CrossAttention`) runs on `d3pm_cross_attention` as well
+        (`attention.fuse_cross_attention`; its head-averaged map, the block's second output, is then None - the
+        denoiser drops it).  Inference only - training, autocast and masked calls still run the reference's modules;
+        `state_dict()` is unchanged.  Composes with `enable_fused_head()` and the one-pass shared conditioning.  After
+        the call the self-attention is fused iff `enable` and the cross-attention iff `enable and cross`: `enable=False`
+        restores the original modules of both kinds."""
         attention.fuse_self_attention(self.transformer, enable)
+        attention.fuse_cross_attention(self.transformer, enable and cross)
         return self
 
     def _head_weights(self) -> "head.HeadWeights":

@@ -371,6 +371,30 @@ typedef struct d3pm_attn_desc {
 
 int d3pm_self_attention(const d3pm_attn_desc* desc);
 
+/* ---------------------------------------------------------------- denoiser cross-attention (SURVEY.md §8 f3)
+ * The cross-attention of the denoiser's blocks, CrossAttention (the blocks' attn2 over the M condition tokens), after its
+ * q / k / v Linears and before `proj`, forward only, fp32:
+ *     y[b*N + n][h*hd + c] = sum_{j < M} softmax_j(scale * q_{b,n,h} . k_{b,j,h}) v_{b,j,h}[c]
+ * with q_{b,n,h} = q[b*N + n][h*hd .. h*hd + hd) and k_{b,j,h} = k[b*M + j][h*hd .. h*hd + hd) (v alike).  q is the output of
+ * `query(x)` ([B*N][pitch_q]); k and v are the outputs of `key(encoder_output)` and `value(encoder_output)` ([B*M][pitch_kv]
+ * each), read in place; y is written as [B*N][pitch_y], the layout `proj` takes.  The numerics of d3pm_self_attention: the
+ * [N, M] scores never leave registers (no workspace), exact running maximum per block of keys, ex2.approx on pre-scaled
+ * scores, Kahan-compensated block sums.  The head-averaged attention map the reference also returns is not produced.
+ * head_dim = 4 only (other values return D3PM_ERR_UNSUPPORTED).  Any N, M >= 1 and B >= 1, heads <= 65535; pointers
+ * 16-byte aligned, pitches % 4 == 0 and >= heads * head_dim.  Launches on `stream` only (CUDA-graph capturable).        */
+typedef struct d3pm_cross_attn_desc {
+  const float* q;      /* [B*N][pitch_q] */
+  const float* k;      /* [B*M][pitch_kv] */
+  const float* v;      /* [B*M][pitch_kv] */
+  float* y;            /* [B*N][pitch_y] out, columns [0, heads * head_dim) written */
+  int32_t B, N, M, heads, head_dim;
+  int64_t pitch_q, pitch_kv, pitch_y; /* in floats, >= heads * head_dim */
+  float scale;         /* softmax scale, 1 / sqrt(head_dim) in the reference */
+  d3pm_stream_t stream;
+} d3pm_cross_attn_desc;
+
+int d3pm_cross_attention(const d3pm_cross_attn_desc* desc);
+
 /* ---------------------------------------------------------------- host-buffer entry points
  * For a caller whose denoiser output lives in HOST memory (the reference's CPU tensors; bench.py's `e2e`): a handle owns
  * the device staging buffers for one batch shape, a copy stream and a compute stream.  `run` copies the inputs up in

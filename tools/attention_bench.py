@@ -1,9 +1,10 @@
-"""The denoiser's self-attention at head dimension 4: the reference's math against `d3pm_self_attention`.
+"""The denoiser's attentions at head dimension 4: the reference's math against `d3pm_self_attention` and
+`d3pm_cross_attention`.
 
-    python tools/attention_bench.py [--iters 20] [--shapes 16x4096,16x1024,1x1024] [--denoiser] [--json out.json]
+    python tools/attention_bench.py [--iters 20] [--shapes 16x4096,16x1024,1x1024] [--denoiser] [--standin] [--json out.json]
 
-Per shape (B videos, N tokens, 16 heads of width 4; q, k, v ~ N(0, 1) from a fixed seed) three arms, each warmed up and
-then timed over `--iters` launches with CUDA events (median reported):
+Per shape (B videos, N tokens, 16 heads of width 4; q, k, v ~ N(0, 1) from a fixed seed) three self-attention arms, each
+warmed up and then timed over `--iters` launches with CUDA events (median reported):
 
   (a) `reference`: FullAttention's own math (transformer_utils.py:52-58): q kᵀ * scale, softmax, att @ v, att.mean(1);
   (b) `sdpa`: torch.nn.functional.scaled_dot_product_attention in fp32, whichever backend torch picks (comparison only);
@@ -12,11 +13,17 @@ then timed over `--iters` launches with CUDA events (median reported):
 Each arm's max error against a float64 restatement on 64 sampled query rows (of max|v|), ms, scores/s, and the fused
 kernel against the exponential floor: B * heads * N² ex2 at 16 MUFU.EX2 per clock per SM.  Each arm's SM clock is the
 median nvidia-smi reports while that arm runs back to back for about a second; the floor uses the fused arm's.  The card's
-name and power limit are printed with them.  For scale, `cross` times the math of the blocks' cross-attention `attn2` over the
-77 condition tokens (left to PyTorch: it forms a [B, 16, N, 77] matrix) at the same B and N.
+name and power limit are printed with them.  The blocks' cross-attention `attn2` over the 77 condition tokens is timed the
+same way in two arms: `cross` is CrossAttention's math in PyTorch (it forms a [B, 16, N, 77] matrix and its head mean),
+`cross_fused` is d3pm_cross_attention, with its scores/s and its fraction of the floor of B * heads * N * 77 ex2.
 
 `--denoiser` (only where the reference is staged): two `Text2ImageTransformer` forwards and one `p_sample_tokens` step at
-config 3 (B = 16, N = 4096, K = 4096) with and without `enable_fused_attention()`.
+config 3 (B = 16, N = 4096, K = 4096) eager, with `enable_fused_attention()` and with `enable_fused_attention(cross=True)`.
+
+`--standin`: one forward of a 19-block self-plus-cross stand-in denoiser (tests/cross_attention_standin.py: n_embd 64, 16
+heads, condition 77 x 512, K = 4096) at config 3 (B = 16, N = 4096), eager, fused self and fused self + cross.  It is not
+the reference's denoiser (no AdaLayerNorm, a plain GELU MLP): it measures what each attention costs in a pass of that shape
+where the reference is not staged.
 """
 from __future__ import annotations
 
@@ -108,9 +115,27 @@ def cross_arm(q, kc, vc):
 
 def float64_rows(q, k, v, rows):
     B, N, C = q.shape
+    M = k.shape[1]
     qs = q[:, rows].double().view(B, len(rows), HEADS, HD).transpose(1, 2)
-    att = torch.softmax((qs @ heads_of(k.double(), B, N).transpose(-2, -1)) / math.sqrt(HD), dim=-1)
-    return (att @ heads_of(v.double(), B, N)).transpose(1, 2).reshape(B, len(rows), C)
+    att = torch.softmax((qs @ heads_of(k.double(), B, M).transpose(-2, -1)) / math.sqrt(HD), dim=-1)
+    return (att @ heads_of(v.double(), B, M)).transpose(1, 2).reshape(B, len(rows), C)
+
+
+def ex2_floor_ms(pairs, mhz):
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    return pairs / (EX2_PER_CLK_PER_SM * sms * mhz * 1e6) * 1e3
+
+
+def timed_arm(fn, rows, want, vmax, iters, pairs):
+    """ms, scores/s, error against float64 (of max|v|) and SM clock of one arm."""
+    with torch.no_grad():
+        y = fn()
+        err = float((y[:, rows].double() - want).abs().max()) / vmax
+        del y
+        ms = time_ms(fn, iters)
+        mhz = sustained_clock_mhz(fn)
+    torch.cuda.empty_cache()
+    return {"ms": ms, "scores_per_s": pairs / (ms * 1e-3), "max_err_of_max_v": err, "sm_clock_mhz": mhz}
 
 
 def bench_shape(B, N, iters):
@@ -128,21 +153,19 @@ def bench_shape(B, N, iters):
     scores = B * HEADS * N * N
     out = {"B": B, "N": N, "heads": HEADS, "head_dim": HD, "scores": scores}
     for name, fn in arms.items():
-        with torch.no_grad():
-            y = fn()
-            err = float((y[:, rows].double() - want).abs().max()) / vmax
-            del y
-            ms = time_ms(fn, iters)
-            mhz = sustained_clock_mhz(fn)
-        out[name] = {"ms": ms, "scores_per_s": scores / (ms * 1e-3), "max_err_of_max_v": err, "sm_clock_mhz": mhz}
-        torch.cuda.empty_cache()
-    kc, vc = (torch.randn(B, 77, HEADS * HD, device="cuda", generator=g) for _ in range(2))
-    with torch.no_grad():
-        cross = lambda: cross_arm(q, kc, vc)  # noqa: E731
-        out["cross"] = {"ms": time_ms(cross, iters), "sm_clock_mhz": sustained_clock_mhz(cross)}
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    floor_ms = scores / (EX2_PER_CLK_PER_SM * sms * out["fused"]["sm_clock_mhz"] * 1e6) * 1e3
+        out[name] = timed_arm(fn, rows, want, vmax, iters, scores)
+    floor_ms = ex2_floor_ms(scores, out["fused"]["sm_clock_mhz"])
     out["fused"].update({"ex2_floor_ms": floor_ms, "fraction_of_ex2_floor": floor_ms / out["fused"]["ms"]})
+    kc, vc = (torch.randn(B, 77, HEADS * HD, device="cuda", generator=g) for _ in range(2))
+    want_c = float64_rows(q, kc, vc, rows)
+    vmax_c = float(vc.abs().max())
+    cross_scores = B * HEADS * N * 77
+    out["cross_scores"] = cross_scores
+    out["cross"] = timed_arm(lambda: cross_arm(q, kc, vc)[0], rows, want_c, vmax_c, iters, cross_scores)
+    out["cross_fused"] = timed_arm(lambda: attention.cross_attention(q, kc, vc, HEADS, 1.0 / math.sqrt(HD)), rows, want_c,
+                                   vmax_c, iters, cross_scores)
+    floor_ms = ex2_floor_ms(cross_scores, out["cross_fused"]["sm_clock_mhz"])
+    out["cross_fused"].update({"ex2_floor_ms": floor_ms, "fraction_of_ex2_floor": floor_ms / out["cross_fused"]["ms"]})
     return out
 
 
@@ -161,14 +184,39 @@ def bench_denoiser(iters):
     cf = torch.zeros(B, 77, 512, device=dev)
     t = torch.full((B,), 50, device=dev, dtype=torch.long)
     res = {"ran": True, "B": B, "N": N, "K": K}
-    for fused in (False, True):
-        ours.enable_fused_attention(fused)
+    for arm, fused, cross in (("eager", False, False), ("fused", True, False), ("fused_self_cross", True, True)):
+        ours.enable_fused_attention(fused, cross=cross)
         with torch.no_grad():
             two = time_ms(lambda: (ours.transformer(x, cond, t), ours.transformer(x, cf, t)), max(3, iters // 4), warmup=1)
             step = time_ms(lambda: ours.p_sample_tokens(x, cond, cf, t), max(3, iters // 4), warmup=1)
-        res["fused" if fused else "eager"] = {"two_forwards_ms": two, "p_sample_tokens_ms": step}
+        res[arm] = {"two_forwards_ms": two, "p_sample_tokens_ms": step}
         torch.cuda.empty_cache()
     ours.enable_fused_attention(False)
+    return res
+
+
+def bench_standin(iters):
+    """One forward of a 19-block self-plus-cross stand-in denoiser at config 3, eager / fused self / fused self + cross."""
+    from d3pm_b200 import attention
+    from tests.cross_attention_standin import CrossStandInDenoiser
+    B, N, K = 16, 4096, 4096
+    torch.manual_seed(0)
+    model = CrossStandInDenoiser(K, N, n_layer=19).cuda().eval()
+    g = torch.Generator(device="cuda").manual_seed(0)
+    x = torch.randint(0, K + 1, (B, N), device="cuda", generator=g)
+    cond = torch.randn(B, 77, 512, device="cuda", generator=g)
+    t = torch.full((B,), 50, device="cuda", dtype=torch.long)
+    res = {"what": "stand-in denoiser (tests/cross_attention_standin.py), not the reference's", "B": B, "N": N, "K": K,
+           "n_layer": 19, "n_embd": 64, "heads": HEADS}
+    n = max(3, iters // 4)
+    with torch.no_grad():
+        fwd = lambda: model(x, cond, t)  # noqa: E731
+        res["eager"] = {"forward_ms": time_ms(fwd, n, warmup=1), "sm_clock_mhz": sustained_clock_mhz(fwd, 3.0)}
+        torch.cuda.empty_cache()
+        attention.fuse_self_attention(model)
+        res["fused_self"] = {"forward_ms": time_ms(fwd, n), "sm_clock_mhz": sustained_clock_mhz(fwd)}
+        attention.fuse_cross_attention(model)
+        res["fused_self_cross"] = {"forward_ms": time_ms(fwd, n), "sm_clock_mhz": sustained_clock_mhz(fwd)}
     return res
 
 
@@ -177,6 +225,7 @@ def main():
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--shapes", default="16x4096,16x1024,1x1024")
     ap.add_argument("--denoiser", action="store_true")
+    ap.add_argument("--standin", action="store_true")
     ap.add_argument("--json", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -192,10 +241,16 @@ def main():
         arm = lambda a: f"{r[a]['ms']:9.3f} ms at {r[a]['sm_clock_mhz']:.0f} MHz (err {r[a]['max_err_of_max_v']:.1e})"  # noqa: E731
         print(f"B={B:2d} N={N:5d}: reference {arm('reference')} | sdpa {arm('sdpa')} | fused {arm('fused')}, "
               f"{f['scores_per_s']:.3e} scores/s, ex2 floor {f['ex2_floor_ms']:.3f} ms = {100 * f['fraction_of_ex2_floor']:.0f} %; "
-              f"cross (77 keys) {r['cross']['ms']:.3f} ms at {r['cross']['sm_clock_mhz']:.0f} MHz")
+              f"cross (77 keys) {arm('cross')}")
+        c = r["cross_fused"]
+        print(f"            cross fused {arm('cross_fused')}, {c['scores_per_s']:.3e} scores/s, "
+              f"ex2 floor {1e3 * c['ex2_floor_ms']:.1f} us = {100 * c['fraction_of_ex2_floor']:.0f} %")
     if args.denoiser:
         result["denoiser"] = bench_denoiser(args.iters)
         print("denoiser:", json.dumps(result["denoiser"]))
+    if args.standin:
+        result["standin"] = bench_standin(args.iters)
+        print("stand-in:", json.dumps(result["standin"]))
     if args.json:
         with open(args.json, "w") as fh:
             json.dump(result, fh, indent=1)
